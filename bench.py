@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference-semantics CPU path (oracle)
+    python bench.py ... --dump-outputs DIR    # also save what the last timed step computed, as DIR/*.npy
 
 Headline workload (BASELINE.json configs[1], "cfg2"): ComplEx k=200 (row = 400 fp32), eta=10,
 self-adversarial loss (margin 3, alpha 0.5), Adam lr 1e-3, FB15K-237-shaped synthetic KG
@@ -489,6 +490,23 @@ def extra_sharded(name, dev, rank, world, flush, peak, n_ent=None, steps=5, warm
     return out
 
 
+def dump_outputs(out_dir, eng, loss_before_last, world, rank):
+    """Save what the timed path hands its caller after the last timed step, so that two builds can be compared output
+    for output on identical inputs: both embedding tables (dense [rows, internal_k] float32, as get_embeddings returns
+    them) and that step's [batch loss, regulariser loss] (float64, summed over ranks).  23.6 MB in all for cfg2."""
+    import torch.distributed as dist
+    last = eng.loss_acc - loss_before_last
+    if world > 1:
+        dist.all_reduce(last)
+    if rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    ent, rel = (x.cpu().numpy() for x in eng.get_embeddings())
+    np.save(os.path.join(out_dir, "ent_embeddings.npy"), ent)
+    np.save(os.path.join(out_dir, "rel_embeddings.npy"), rel)
+    np.save(os.path.join(out_dir, "last_step_loss.npy"), last.cpu().numpy())
+
+
 def guarded(extra, key, fn):
     try:
         t0 = time.perf_counter()
@@ -572,11 +590,15 @@ def main_ours(args):
     for i in range(args.steps):
         if os.environ.get("KGE_BENCH_NOFLUSH") != "1":  # (diagnostic switch; the reported numbers always flush)
             flush.fill_(i & 0xff)  # evict L2 (126 MB) outside the timed events
+        if args.dump_outputs and i == args.steps - 1:
+            loss_before_last = eng.loss_acc.clone()  # outside the step's events, like the flush
         step(args.warmup + i, evs[i])
     g1.record()
     cpu_enqueue_ms = 1e3 * (time.perf_counter() - c0) / args.steps  # host time to enqueue one step (flush included)
     sync_all()
     gpu_timeline_ms = g0.elapsed_time(g1) / args.steps                # device time per step, flush included
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, loss_before_last, world, rank)
     launches = eng.launches - launches0
     clocks = sampler.stop() if rank == 0 else None
     if os.environ.get("KGE_BENCH_DEBUG") == "1" and rank == 0:
@@ -776,7 +798,11 @@ if __name__ == "__main__":
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra block (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, save the embedding tables and the loss of the last timed step as DIR/*.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours (the reference arm samples its batch to fit a time budget)")
     if a.impl == "reference":
         main_reference(a)
     else:
